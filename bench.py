@@ -3,7 +3,7 @@
 Llama-3-8B bf16, 1xB200, batch=128 concurrent `analyze` ReAct steps over synthetic Pod YAML
 (P=1536 prompt tokens, G=256 generated tokens, mean decode context 1664; SURVEY.md §8d config 2).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one decode forward of the whole batch (128 sequences, one new token each) through the hot path.
   value  : decode tokens/s, whole job (all N GPUs), inputs resident in HBM, K steps inside one CUDA-event bracket
@@ -21,6 +21,7 @@ N>=2 additionally runs, AFTER the headline (metric/value unchanged), the tensor-
               1.08M-token prefill) at N=8, Llama-3-8B TP=2 at N=2 — decode ms/step, tokens/s per group and per GPU, fraction of the per-GPU
               HBM roofline, the all-reduce chain (in-situ us per all-reduce x count per step).
 `--impl reference` times the CPU port alone (rank 0 only), same JSON line shape.
+`--dump-outputs DIR` writes what the last timed decode step computed (rank 0) as DIR/<name>.npy, see dump_outputs().
 """
 import argparse
 import json
@@ -404,24 +405,26 @@ def run_ours(args, rank, world, local_rank):
             print(json.dumps({"react": rb}), flush=True)
         return
     K, W = args.steps, max(args.warmup, 3)
-    eng = Engine({"model": MODEL, "device": local_rank, "kv_gb": args.kv_gb, "max_batch": BATCH, "max_seq_len": 2048,
+    # context chosen so that the mean over the K timed steps is MEAN_CTX (=P+G/2); a long run gets the sequence length it needs
+    ctx0 = max(64, MEAN_CTX - W - K // 2)
+    eng = Engine({"model": MODEL, "device": local_rank, "kv_gb": args.kv_gb, "max_batch": BATCH, "max_seq_len": max(2048, (ctx0 + K + W + 64) // 64 * 64),
                   "max_step_tokens": 8192, "seed": 1234, "tokenizer": TOKENIZER,
                   "prefix_cache": 0,       # every timed prompt token is really prefilled: no cached outputs inside the timed region
                   **json.loads(args.engine_extra)})
     info = eng.info
     # ------------------------------------------------------------------ value: device-resident decode steps
-    # context chosen so that the mean over the K timed steps is MEAN_CTX (=P+G/2)
-    ctx0 = max(64, MEAN_CTX - W - K // 2)
     # ONE sampler for the whole job (rank 0, all N GPUs): NVML queries take driver-wide locks; N polling processes are the
     # suspected source of the host gaps seen at N=4 (0.5 ms per 8.5 ms step against 0.02 ms at N=1) and one is enough anyway
     clocks = ClockSampler(",".join(str(i) for i in range(world)), 200 if world == 1 else 500) if rank == 0 else None
     if clocks:
         clocks.start()
     barrier()
-    r = eng.bench_decode(BATCH, ctx0, K, W)
+    r = eng.bench_decode(BATCH, ctx0, K, W, last_outputs=bool(args.dump_outputs))
     barrier()
     clk = clocks.stop() if clocks else None
     ms_step = allmax(r["ms_per_step"])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r)
     value = world * BATCH / (ms_step / 1e3)
     # ------------------------------------------------------------------ roofline: dominant kernel (decode attention)
     os.environ["OA_PROFILE_ATTN"] = "1"
@@ -534,6 +537,23 @@ def run_ours(args, rank, world, local_rank):
         dist.barrier(); dist.destroy_process_group()
 
 
+DUMP_LOGIT_COLUMNS = 32768
+
+
+def dump_outputs(out_dir, r):
+    """What the last timed decode step computed, so that two builds can be compared output for output on identical inputs (seeded
+    weights, seeded prompt ids): every sequence's next-token id, the logit it won with, and the fp32 logits at a fixed seeded sample
+    of vocabulary columns (all 128 x 128,256 of them would be 66 MB)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    ids, logits = r["last_ids"], r["last_logits"]
+    cols = np.sort(np.random.default_rng(0).choice(logits.shape[1], size=min(DUMP_LOGIT_COLUMNS, logits.shape[1]), replace=False))
+    arrays = {"decode_next_token_ids": ids.astype(np.float64), "decode_next_token_logit": logits[np.arange(len(ids)), ids],
+              "decode_logits_sample": logits[:, cols], "decode_logits_sample_columns": cols.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def cpu_baseline(n_decode=24, n_prompt=32, ctx=MEAN_CTX, repeats=3):
     """The oracle (CPU port of the same decoder, same seeded 8B weights) on the host cores: B=1 (a single-slot local server), decode steps
     at the BENCHMARK's context length — the cache positions [0, ctx) are filled with seeded values (oracle fill_kv: a timing aid, a CPU
@@ -587,7 +607,7 @@ def run_reference(args, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=64)
+    ap.add_argument("--steps", type=int, default=64, help="timed decode steps of the headline")
     ap.add_argument("--warmup", type=int, default=8)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--kv-gb", type=float, default=60.0, dest="kv_gb")
@@ -608,7 +628,11 @@ def main():
     ap.add_argument("--engine-extra", default="{}", dest="engine_extra", help="dev: JSON of engine options merged into the config (A/B runs)")
     ap.add_argument("--tp-deadline", type=float, default=900.0, dest="tp_deadline")
     ap.add_argument("--tp-only", action="store_true", help="dev: only the tensor-parallel block (prints {\"tp\": ...}; NOT a bench line)")
+    ap.add_argument("--dump-outputs", default="", dest="dump_outputs", metavar="DIR",
+                    help="write what the last timed decode step computed as DIR/<name>.npy (float32/float64; that one step also stores its logits)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":

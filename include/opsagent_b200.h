@@ -127,6 +127,10 @@ OA_API int oa_debug_prefill_logits(oa_engine*, const int32_t* tokens, int32_t n,
  * timed steps, out[4]=attention-kernel ms/step (avg), out[5]=algorithmic bytes/step,
  * out[6]=sum of per-step device durations / steps (host gaps excluded) */
 OA_API int oa_bench_decode(oa_engine*, int32_t batch, int32_t ctx_len, int32_t steps, int32_t warmup, double* out, int32_t n_out);
+/* the same, plus what the last timed step computed: next-token ids -> last_ids[batch] and, when last_logits is not NULL, its fp32
+ * logits -> last_logits[batch, vocab] (that one step then also stores them; its ids are unchanged).  Either pointer may be NULL. */
+OA_API int oa_bench_decode_ex(oa_engine*, int32_t batch, int32_t ctx_len, int32_t steps, int32_t warmup, double* out, int32_t n_out,
+                              int32_t* last_ids, float* last_logits);
 
 /* in-situ per-kernel-class timings accumulated while OA_PROFILE_ALL=1 (JSON name -> [total ms, launches]) */
 OA_API int oa_debug_kernel_times(oa_engine*, char* buf, size_t n, int32_t reset);

@@ -32,7 +32,7 @@ class OaChatResp(C.Structure):
 SYMBOLS = [
     "oa_engine_create", "oa_engine_destroy", "oa_chat_complete", "oa_chat_submit", "oa_chat_wait", "oa_free_resp",
     "oa_tokens_submit", "oa_count_tokens", "oa_apply_chat_template", "oa_last_error", "oa_engine_stats", "oa_model_info",
-    "oa_debug_prefill_logits", "oa_bench_decode", "oa_k_rmsnorm", "oa_k_gemm", "oa_k_init_weight", "oa_k_paged_attention",
+    "oa_debug_prefill_logits", "oa_bench_decode", "oa_bench_decode_ex", "oa_k_rmsnorm", "oa_k_gemm", "oa_k_init_weight", "oa_k_paged_attention",
     "oa_kernel_launches", "oa_version", "oa_host_apply_chat_template", "oa_host_decode_plan", "oa_host_streamk_plan", "oa_host_bpe_encode", "oa_host_bpe_decode", "oa_host_model_info",
     "oa_k_gemm_streamk", "oa_debug_kernel_times", "oa_engine_serve", "oa_host_grammar_step", "oa_host_grammar_step_ex", "oa_host_grammar_token_mask", "oa_http_start", "oa_http_port", "oa_http_stats", "oa_http_stop", "oa_http_last_error", "oa_host_json_roundtrip", "oa_chat_cancel", "oa_chat_submit_ex", "oa_chat_wait_ex",
 ]
@@ -67,6 +67,7 @@ def load() -> C.CDLL:
     L.oa_model_info.argtypes = [vp, C.c_char_p, C.c_size_t]; L.oa_model_info.restype = C.c_int
     L.oa_debug_prefill_logits.argtypes = [vp, vp, i32, vp]; L.oa_debug_prefill_logits.restype = C.c_int
     L.oa_bench_decode.argtypes = [vp, i32, i32, i32, i32, C.POINTER(C.c_double), i32]; L.oa_bench_decode.restype = C.c_int
+    L.oa_bench_decode_ex.argtypes = [vp, i32, i32, i32, i32, C.POINTER(C.c_double), i32, vp, vp]; L.oa_bench_decode_ex.restype = C.c_int
     L.oa_k_rmsnorm.argtypes = [vp, vp, vp, i32, i32, f32, vp]; L.oa_k_rmsnorm.restype = C.c_int
     L.oa_k_gemm.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp]; L.oa_k_gemm.restype = C.c_int
     L.oa_k_gemm_streamk.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, vp]; L.oa_k_gemm_streamk.restype = C.c_int

@@ -181,7 +181,9 @@ public:
         return OA_OK;
     }
 
-    int bench_decode(int batch, int ctx_len, int steps, int warmup, double* out, int n_out) {
+    // last_ids [batch] / last_logits [batch, vocab] (host, optional): what the last timed step computed; asking for the logits makes
+    // that one step also store them (the arg-max it returns is unchanged)
+    int bench_decode(int batch, int ctx_len, int steps, int warmup, double* out, int n_out, int32_t* last_ids = nullptr, float* last_logits = nullptr) {
         if (batch <= 0 || batch > opt_.max_batch || ctx_len <= 0 || ctx_len + steps + warmup + 1 > opt_.max_seq_len || n_out < 6)
             return fail(OA_ERR_BAD_REQUEST, "bench_decode: batch <= max_batch, ctx_len+steps+warmup < max_seq_len, n_out >= 6");
         std::lock_guard<std::mutex> step(step_mu_);
@@ -233,6 +235,8 @@ public:
             model_.profile_all = prof_all;
             std::vector<int32_t> last(batch);
             for (int b = 0; b < batch; ++b) last[b] = synth(b, P);
+            float* d_logits = nullptr;
+            if (last_logits) cuda_check(cudaMalloc(&d_logits, (size_t)batch * V * 4), "cudaMalloc logits");
             double ctx_sum = 0; float total_ms = 0; uint64_t launches0 = 0;
             cudaEvent_t eb0, eb1; cudaEventCreate(&eb0); cudaEventCreate(&eb1);
             model_.attn_ms_accum = 0;
@@ -250,8 +254,10 @@ public:
                     launches0 = launches_total(); model_.attn_ms_accum = 0; cudaEventRecord(eb0, model_.stream);
                 }
                 const bool timed = it >= warmup;
+                float* step_logits = it == warmup + steps - 1 ? d_logits : nullptr;
+                in.want_logits = step_logits != nullptr;
                 if (timed) { cudaEventRecord(e0, model_.stream); ctx_sum += pos + 1; }
-                run_forward(in, nullptr);
+                run_forward(in, step_logits);
                 if (timed) cudaEventRecord(e1, model_.stream);
                 model_.sync();
                 if (timed) { float ms = 0; cudaEventElapsedTime(&ms, e0, e1); total_ms += ms; }
@@ -262,7 +268,11 @@ public:
             float bracket_ms = 0; cudaEventElapsedTime(&bracket_ms, eb0, eb1);
             const uint64_t launches1 = launches_total();
             cudaEventDestroy(e0); cudaEventDestroy(e1); cudaEventDestroy(eb0); cudaEventDestroy(eb1);
+            if (last_ids) std::copy(last.begin(), last.end(), last_ids);
+            cudaError_t le = cudaSuccess;
+            if (d_logits) { le = cudaMemcpy(last_logits, d_logits, (size_t)batch * V * 4, cudaMemcpyDeviceToHost); cudaFree(d_logits); }
             { std::lock_guard<std::mutex> lk(mu_); for (auto& pv : pages) for (int p : pv) release_page_locked(p); }
+            cuda_check(le, "logits D2H");
             const double mean_ctx = ctx_sum / steps;
             out[0] = bracket_ms / steps; if (n_out > 6) out[6] = total_ms / steps; out[1] = prefill_ms; out[2] = (double)(launches1 - launches0) / steps; out[3] = mean_ctx;
             out[4] = model_.profile_attn ? model_.attn_ms_accum / steps : 0.0;
@@ -777,15 +787,19 @@ int oa_debug_prefill_logits(oa_engine* h, const int32_t* tokens, int32_t n, floa
     if (!h || !tokens || !logits_out) return fail(OA_ERR_BAD_REQUEST, "null argument");
     return h->e->debug_prefill_logits(tokens, n, logits_out);
 }
-int oa_bench_decode(oa_engine* h, int32_t batch, int32_t ctx_len, int32_t steps, int32_t warmup, double* out, int32_t n_out) {
+int oa_bench_decode_ex(oa_engine* h, int32_t batch, int32_t ctx_len, int32_t steps, int32_t warmup, double* out, int32_t n_out,
+                       int32_t* last_ids, float* last_logits) {
     if (!h || !out) return fail(OA_ERR_BAD_REQUEST, "null argument");
     const char* pa = std::getenv("OA_PROFILE_ATTN");
     h->e->model().profile_attn = pa && pa[0] == '1';
     const char* pall = std::getenv("OA_PROFILE_ALL");
     h->e->model().profile_all = pall && pall[0] == '1';
-    int rc = h->e->bench_decode(batch, ctx_len, steps, warmup, out, n_out);
+    int rc = h->e->bench_decode(batch, ctx_len, steps, warmup, out, n_out, last_ids, last_logits);
     h->e->model().profile_attn = false; h->e->model().profile_all = false;
     return rc;
+}
+int oa_bench_decode(oa_engine* h, int32_t batch, int32_t ctx_len, int32_t steps, int32_t warmup, double* out, int32_t n_out) {
+    return oa_bench_decode_ex(h, batch, ctx_len, steps, warmup, out, n_out, nullptr, nullptr);
 }
 int oa_debug_kernel_times(oa_engine* h, char* buf, size_t n, int32_t reset) {
     if (!h || !buf) return fail(OA_ERR_BAD_REQUEST, "null argument");

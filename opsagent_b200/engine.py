@@ -149,8 +149,16 @@ class Engine:
         _check(self._L.oa_debug_kernel_times(self._h, buf, 4096, int(reset)))
         return json.loads(buf.value.decode())
 
-    def bench_decode(self, batch: int, ctx_len: int, steps: int, warmup: int) -> dict:
+    def bench_decode(self, batch: int, ctx_len: int, steps: int, warmup: int, last_outputs: bool = False) -> dict:
+        """last_outputs: also return what the last timed step computed, "last_ids" (int32 [batch]) and "last_logits" (fp32 [batch, vocab])"""
+        import numpy as np
         out = (C.c_double * 8)()
-        _check(self._L.oa_bench_decode(self._h, batch, ctx_len, steps, warmup, out, 8))
-        return {"ms_per_step": out[0], "prefill_ms": out[1], "launches_per_step": out[2], "mean_ctx": out[3],
-                "attn_ms_per_step": out[4], "algorithmic_bytes_per_step": out[5], "device_ms_per_step": out[6]}
+        ids = np.zeros(batch, np.int32) if last_outputs else None
+        logits = np.zeros((batch, self.info["vocab"]), np.float32) if last_outputs else None
+        _check(self._L.oa_bench_decode_ex(self._h, batch, ctx_len, steps, warmup, out, 8, None if ids is None else ids.ctypes.data,
+                                          None if logits is None else logits.ctypes.data))
+        r = {"ms_per_step": out[0], "prefill_ms": out[1], "launches_per_step": out[2], "mean_ctx": out[3],
+             "attn_ms_per_step": out[4], "algorithmic_bytes_per_step": out[5], "device_ms_per_step": out[6]}
+        if last_outputs:
+            r["last_ids"], r["last_logits"] = ids, logits
+        return r

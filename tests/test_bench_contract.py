@@ -68,6 +68,29 @@ def test_our_arm_line(name):
     assert r["traffic"] is None or r["traffic"] >= 0.9 * r["algorithmic_bytes_per_launch"]
 
 
+def test_dump_outputs_are_float_files_within_64mb(tmp_path):
+    """--dump-outputs DIR: float32/float64 .npy files, at most 64 MB in all, the same logit columns on every run"""
+    import sys
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(3)
+    logits = rng.standard_normal((bench.BATCH, 128256), dtype=np.float32)
+    r = {"last_ids": logits.argmax(1).astype(np.int32), "last_logits": logits}
+    bench.dump_outputs(str(tmp_path / "a"), r)
+    bench.dump_outputs(str(tmp_path / "b"), r)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files and all(f.endswith(".npy") for f in files)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 * 10 ** 6
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), f
+    ids, top = np.load(tmp_path / "a" / "decode_next_token_ids.npy"), np.load(tmp_path / "a" / "decode_next_token_logit.npy")
+    assert np.array_equal(ids, r["last_ids"]) and np.array_equal(top, logits.max(1))
+    cols = np.load(tmp_path / "a" / "decode_logits_sample_columns.npy").astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "a" / "decode_logits_sample.npy"), logits[:, cols])
+
+
 @pytest.mark.parametrize("ref,ours_name", [("r01h_bench_reference_arm.json", "r01h_bench.json"), ("r02h_bench_reference_arm.json", "r02h_bench.json")])
 def test_reference_arm_line(ref, ours_name):
     line = load(ref)

@@ -611,6 +611,29 @@ def test_benchmarked_batch_geometry_matches_oracle():
     print(f"batch geometry: {checked} sequences checked, {same}/{checked * G} tokens identical")
 
 
+def test_bench_decode_hands_back_what_its_last_step_computed():
+    """bench.py --dump-outputs: the last timed step's logits match the oracle on the same seeded prompt ids, its next-token ids are their
+    arg-max, and two runs with the same arguments agree bit for bit (two builds are compared on these outputs)."""
+    spec, eng = make_engine("tiny-llama-d128")
+    B, ctx, V = 8, 100, spec.vocab
+
+    def synth(b, i):          # the seeded prompt ids of bench_decode (engine.cpp)
+        h = ((b + 1) * 0x9E3779B97F4A7C15 + i * 0xBF58476D1CE4E5B9) & (2 ** 64 - 1)
+        return (h ^ (h >> 29)) % V
+    one = eng.bench_decode(B, ctx, 1, 0, last_outputs=True)          # one decode step: input synth(b, ctx-1) at position ctx-1
+    orc = O.Oracle(spec, max_pos=512, mode=1)
+    for b in range(B):
+        ref = orc.forward(np.array([synth(b, i) for i in range(ctx)], np.int32))[0]
+        assert np.abs(one["last_logits"][b] - ref).max() < LOGIT_TOL, b
+    orc.close()
+    r1 = eng.bench_decode(B, ctx, 3, 2, last_outputs=True)
+    r2 = eng.bench_decode(B, ctx, 3, 2, last_outputs=True)
+    assert np.isfinite(r1["last_logits"]).all() and (r1["last_ids"] == r1["last_logits"].argmax(1)).all()
+    assert np.array_equal(r1["last_ids"], r2["last_ids"]) and np.array_equal(r1["last_logits"], r2["last_logits"])
+    assert eng.stats()["pages_free"] == eng.stats()["pages_total"]
+    eng.close()
+
+
 @pytest.mark.parametrize("name", CASES + ["tiny-llama-8bheads", "llama-3.2-1b"])
 def test_cluster_splitk_projections_match_oracle_and_streamk(name):
     """sk_clusterk=7: qkv (+bias, RoPE, paged-KV write), o and down (+residual) as cluster split-K GEMMs with the reduction through distributed

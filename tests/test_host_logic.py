@@ -499,20 +499,20 @@ PROMPTS_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden",
 
 
 def test_prompt_fixtures_are_the_reference_constants_verbatim():
-    """byte lengths are the ones SURVEY.md §8a measured (3,233 / 3,109 / 1,965 / 2,164 B); sha256 pins every byte; when the reference
-    tree is present (build container) the fixtures are re-extracted and compared"""
+    """byte lengths are the ones SURVEY.md §8a measured (3,233 / 3,109 / 1,965 / 2,164 B); index.json holds the byte length and sha256
+    of every constant as extract_prompts.py read it from the reference's sources, so every fixture byte is pinned to that extraction"""
     idx = json.load(open(os.path.join(PROMPTS_DIR, "index.json")))
+    sys.path.insert(0, PROMPTS_DIR)
+    import extract_prompts
+    assert set(idx) == set(extract_prompts.SOURCES) | set(extract_prompts.SYSTEM_LINES)
+    for name, (rel, *_rest) in {**extract_prompts.SOURCES, **extract_prompts.SYSTEM_LINES}.items():
+        assert idx[name]["source"].split(":")[0] == rel, name
     want = {"executeSystemPrompt_cn": 3233, "diagnoseSystemPrompt": 3109, "analysisPrompt": 1965, "auditPrompt": 2164}
     for name, meta in idx.items():
         raw = open(os.path.join(PROMPTS_DIR, name + ".txt"), "rb").read()
         assert len(raw) == meta["bytes"] and hashlib.sha256(raw).hexdigest() == meta["sha256"], name
         if name in want:
             assert len(raw) == want[name]
-    if os.path.isdir("/root/reference/pkg"):
-        sys.path.insert(0, PROMPTS_DIR)
-        import extract_prompts
-        for name, (text, _where, _use) in extract_prompts.extract("/root/reference").items():
-            assert open(os.path.join(PROMPTS_DIR, name + ".txt"), "rb").read() == text.encode("utf-8"), name
 
 
 def test_toolprompt_marshal_is_go_json_marshal_byte_for_byte():
