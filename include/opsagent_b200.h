@@ -148,6 +148,37 @@ OA_API int oa_k_init_weight(void* dst, uint64_t seed, uint64_t tensor_id, int64_
 OA_API int oa_k_paged_attention(const void* q, void* out, const void* kv_cache, int32_t num_pages, const int32_t* block_tables,
                          int32_t max_pages_per_seq, const int32_t* ctx_lens, const int32_t* q_lens, int32_t n_seqs,
                          int32_t n_heads, int32_t n_kv, int32_t head_dim, int32_t force_splits, void* stream);
+/* the same on one layer of a cache [n_layers][2][num_pages][n_kv][64][D], with the decode plan's CTA target (<= 0: two per SM, the
+ * engine's default) and, for decode, the merge: merge_counters NULL = separate merge kernel, else a device int32 array with one counter
+ * per cut (sequence, kv head) item, zeroed once by the caller — the kernel merges in place and each call advances an item's counter by its
+ * piece count (the engine's per-layer use within one step) */
+OA_API int oa_k_paged_attention_ex(const void* q, void* out, const void* kv_cache, int32_t num_pages, int32_t n_layers, int32_t layer,
+                                   const int32_t* block_tables, int32_t max_pages_per_seq, const int32_t* ctx_lens, const int32_t* q_lens,
+                                   int32_t n_seqs, int32_t n_heads, int32_t n_kv, int32_t head_dim, int32_t force_splits, int32_t n_ctas_target,
+                                   int32_t* merge_counters, void* stream);
+/* Decode projections (M <= 128) with their fused epilogues, launched as the engine launches them.  All pointers are device pointers;
+ * B is the [N, K] weight; tile_flags = caller-owned zeroed uint32 counters (>= N/128), which the fused kernels leave zeroed again.
+ * o / down: x[M, ldx] += A.B^T (bf16, in place), then xn[M, N] = rmsnorm(x) * gain.
+ *   path 0: stream-K GEMM + sum/residual/norm consumer (default); 1: stream-K GEMM finishing the residual + norm kernel;
+ *   2: cluster split-K GEMM with `cluster` CTAs per tile + norm kernel.  xn NULL (paths 1, 2) skips the norm; with a norm, ldx == N. */
+OA_API int oa_k_sk_resid_rmsnorm(int32_t path, const void* A, const void* B, int32_t M, int32_t N, int32_t K, int32_t n_ctas, int32_t cluster,
+                                 void* x, int32_t ldx, const void* gain, void* xn, float eps, uint32_t* tile_flags, void* stream);
+/* gate/up: B = [2F, K] with rows interleaved 16 gate / 16 up; act[M, F] = silu(gate) * up.
+ *   path 0: stream-K GEMM + SwiGLU consumer; 1: stream-K GEMM finishing the SwiGLU (default). */
+OA_API int oa_k_sk_swiglu(int32_t path, const void* A, const void* B, int32_t M, int32_t F, int32_t K, int32_t n_ctas, void* act,
+                          uint32_t* tile_flags, void* stream);
+/* qkv: B = [(nh + 2 nkv) D, K], optional bias; rows -> (+ bias) -> bf16 -> RoPE at positions[M] -> q_out[M, nh*D] and the K/V rows of
+ * slots[M] in layer `layer` of kv_cache [n_layers][2][num_pages][nkv][64][D].  rope_cos/sin: [max_pos, D/2] fp32.
+ *   path 0: stream-K GEMM + RoPE/KV consumer (default); 1: stream-K GEMM finishing RoPE + KV write; 2: cluster split-K GEMM with
+ *   `cluster` CTAs per tile; 3: tile GEMM (bf16 qkv + bias) + RoPE/KV kernel (the prefill path). */
+OA_API int oa_k_qkv_rope(int32_t path, const void* A, const void* B, int32_t M, int32_t K, int32_t n_ctas, int32_t cluster, const void* bias,
+                         const int32_t* positions, const int32_t* slots, const float* rope_cos, const float* rope_sin, void* q_out,
+                         void* kv_cache, int32_t num_pages, int32_t n_layers, int32_t layer, int32_t nh, int32_t nkv, int32_t D,
+                         uint32_t* tile_flags, void* stream);
+/* LM head: logits[M, N] fp32 (optional) and ids[M] = per-row arg-max (ties -> lowest column).  Rows with mask_slot[r] >= 0 take the
+ * arg-max only over columns c whose bit col_offset + c is set in mask_table[mask_slot[r] * mask_words ...]; ids are shard-local columns. */
+OA_API int oa_k_lm_head(const void* A, const void* B, int32_t M, int32_t N, int32_t K, int32_t block_n, const uint32_t* mask_table,
+                        const int32_t* mask_slot, int32_t mask_words, int32_t col_offset, float* logits, int32_t* ids, void* stream);
 /* ---- host-only logic, callable without a GPU (CPU tests) ---- */
 /* chat template + tokenizer of the model described by config_json */
 OA_API int oa_host_apply_chat_template(const char* config_json, const oa_msg* msgs, int32_t n_msgs, int32_t* out_ids, int32_t cap, int32_t* n_out);
@@ -164,6 +195,8 @@ OA_API int oa_host_decode_plan(const int32_t* ctx_lens, int32_t n_seqs, int32_t 
 OA_API int oa_host_streamk_plan(int32_t N, int32_t K, int32_t block_n, int32_t n_ctas, int64_t* cta_unit0_out, int32_t cap_ctas,
                          int32_t* tile_first_out, int32_t* tile_last_out, int32_t cap_tiles, int32_t* n_ctas_out, int32_t* n_tiles_out,
                          int32_t* kb_out);
+/* cluster size (8, 4, 3, 2) the decode path would give the cluster split-K GEMM of an N x K projection on `sms` SMs, or 0 (keep stream-K) */
+OA_API int32_t oa_host_clusterk_pick(int32_t N, int32_t K, int32_t sms, int32_t min_fill_pct);
 /* byte-level BPE tokenizer read from a Hugging Face tokenizer.json (Llama-3 / Qwen2.5 format), host only: what the engine uses
  * for text when its config names one ("tokenizer": path) instead of the synthetic byte-level vocabulary.  Loaded files are cached
  * by path.  encode: *n_out = number of ids (written up to cap; OA_ERR_BAD_REQUEST if cap is too small or the file is unsupported);

@@ -35,6 +35,7 @@ SYMBOLS = [
     "oa_debug_prefill_logits", "oa_bench_decode", "oa_bench_decode_ex", "oa_k_rmsnorm", "oa_k_gemm", "oa_k_init_weight", "oa_k_paged_attention",
     "oa_kernel_launches", "oa_version", "oa_host_apply_chat_template", "oa_host_decode_plan", "oa_host_streamk_plan", "oa_host_bpe_encode", "oa_host_bpe_decode", "oa_host_model_info",
     "oa_k_gemm_streamk", "oa_debug_kernel_times", "oa_engine_serve", "oa_host_grammar_step", "oa_host_grammar_step_ex", "oa_host_grammar_token_mask", "oa_http_start", "oa_http_port", "oa_http_stats", "oa_http_stop", "oa_http_last_error", "oa_host_json_roundtrip", "oa_chat_cancel", "oa_chat_submit_ex", "oa_chat_wait_ex",
+    "oa_k_paged_attention_ex", "oa_k_sk_resid_rmsnorm", "oa_k_sk_swiglu", "oa_k_qkv_rope", "oa_k_lm_head", "oa_host_clusterk_pick",
 ]
 
 _lib = None
@@ -74,10 +75,18 @@ def load() -> C.CDLL:
     L.oa_debug_kernel_times.argtypes = [vp, C.c_char_p, C.c_size_t, i32]; L.oa_debug_kernel_times.restype = C.c_int
     L.oa_k_init_weight.argtypes = [vp, u64, u64, C.c_int64, C.c_int64, C.c_int64, f32, f32, vp]; L.oa_k_init_weight.restype = C.c_int
     L.oa_k_paged_attention.argtypes = [vp, vp, vp, i32, vp, i32, vp, vp, i32, i32, i32, i32, i32, vp]; L.oa_k_paged_attention.restype = C.c_int
+    L.oa_k_paged_attention_ex.argtypes = [vp, vp, vp, i32, i32, i32, vp, i32, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
+    L.oa_k_paged_attention_ex.restype = C.c_int
+    L.oa_k_sk_resid_rmsnorm.argtypes = [i32, vp, vp, i32, i32, i32, i32, i32, vp, i32, vp, vp, f32, vp, vp]; L.oa_k_sk_resid_rmsnorm.restype = C.c_int
+    L.oa_k_sk_swiglu.argtypes = [i32, vp, vp, i32, i32, i32, i32, vp, vp, vp]; L.oa_k_sk_swiglu.restype = C.c_int
+    L.oa_k_qkv_rope.argtypes = [i32, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
+    L.oa_k_qkv_rope.restype = C.c_int
+    L.oa_k_lm_head.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp, i32, i32, vp, vp, vp]; L.oa_k_lm_head.restype = C.c_int
     L.oa_host_apply_chat_template.argtypes = [C.c_char_p, C.POINTER(OaMsg), i32, vp, i32, C.POINTER(i32)]; L.oa_host_apply_chat_template.restype = C.c_int
     L.oa_host_bpe_encode.argtypes = [C.c_char_p, C.c_char_p, i32, vp, i32, C.POINTER(i32)]; L.oa_host_bpe_encode.restype = C.c_int
     L.oa_host_bpe_decode.argtypes = [C.c_char_p, vp, i32, vp, i32, C.POINTER(i32)]; L.oa_host_bpe_decode.restype = C.c_int
     L.oa_host_streamk_plan.argtypes = [i32, i32, i32, i32, vp, i32, vp, vp, i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]; L.oa_host_streamk_plan.restype = C.c_int
+    L.oa_host_clusterk_pick.argtypes = [i32, i32, i32, i32]; L.oa_host_clusterk_pick.restype = i32
     L.oa_host_decode_plan.argtypes = [vp, i32, i32, i32, i32, vp, i32, vp, i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]; L.oa_host_decode_plan.restype = C.c_int
     L.oa_host_grammar_step.argtypes = [i32, vp, i32, vp, C.POINTER(i32)]; L.oa_host_grammar_step.restype = C.c_int
     L.oa_host_grammar_step_ex.argtypes = [i32, C.c_char_p, vp, i32, vp, C.POINTER(i32)]; L.oa_host_grammar_step_ex.restype = C.c_int

@@ -27,6 +27,17 @@ struct DevBuf {
     ~DevBuf() { if (p) cudaFree(p); }
 };
 int rc_of(cudaError_t e) { return e == cudaSuccess ? OA_OK : OA_ERR_INTERNAL; }
+int device_sm_count() {
+    int dev = 0, n = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
+    return n;
+}
+// A [M,K] and B [N,K] as the decode projections map them: A in 128-row boxes, B in 128-column tiles (BN = 128, the engine's stream-K tile)
+bool proj_maps(const void* A, const void* B, int M, int N, int K, CUtensorMap& tmA, CUtensorMap& tmB) {
+    return make_tmap_bf16_2d(&tmA, A, (uint64_t)M, (uint64_t)K, (uint64_t)K, 128, 64) == 0 &&
+           make_tmap_bf16_2d(&tmB, B, (uint64_t)N, (uint64_t)K, (uint64_t)K, 128, 64) == 0;
+}
 }  // namespace
 
 // test-only: materialise the deterministic fixed-order sum of stream-K partials as fp32 [M,N]
@@ -88,14 +99,125 @@ int oa_k_gemm(const void* A, const void* B, int32_t M, int32_t N, int32_t K, int
     return rc_of(launch_gemm(&tmA, &tmB, p, epilogue, block_n, s));
 }
 
+// ---- the decode step's projections with their epilogues, each through the launcher pairing DeviceModel::forward uses ----
+int oa_k_sk_resid_rmsnorm(int32_t path, const void* A, const void* B, int32_t M, int32_t N, int32_t K, int32_t n_ctas, int32_t cluster,
+                          void* x, int32_t ldx, const void* gain, void* xn, float eps, uint32_t* tile_flags, void* stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    if (M <= 0 || M > 128 || N <= 0 || K <= 0 || n_ctas <= 0 || path < 0 || path > 2) return OA_ERR_BAD_REQUEST;
+    if ((path == 0 || xn) && ldx != N) return OA_ERR_BAD_REQUEST;          // the norm kernels read x with row stride N
+    if (path == 0 && !xn) return OA_ERR_BAD_REQUEST;
+    if (path == 2 && (K + 63) / 64 < cluster) return OA_ERR_BAD_REQUEST;     // every cluster rank needs at least one k-block
+    CUtensorMap tmA, tmB;
+    if (!proj_maps(A, B, M, N, K, tmA, tmB)) return OA_ERR_INTERNAL;
+    DevBuf ws(path == 2 ? 16 : streamk_ws_bytes(N, 128, n_ctas, 128));
+    if (!ws.p) return OA_ERR_INTERNAL;
+    const StreamK sk = make_streamk((float*)ws.p, N, K, 128, n_ctas, 128);
+    cudaError_t e;
+    if (path == 0) {
+        e = launch_gemm_streamk(&tmA, &tmB, M, N, K, sk, s);
+        if (e == cudaSuccess) e = launch_sk_resid_rmsnorm(sk, x, gain, xn, M, N, eps, s);
+    } else {
+        e = path == 1 ? launch_gemm_streamk_resid(&tmA, &tmB, M, N, K, sk, x, ldx, tile_flags, s)
+                      : launch_gemm_clusterk_resid(&tmA, &tmB, M, N, K, cluster, x, ldx, s);
+        if (e == cudaSuccess && xn) e = launch_rmsnorm_wide(x, gain, xn, M, N, eps, s);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    return rc_of(e);
+}
+
+int oa_k_sk_swiglu(int32_t path, const void* A, const void* B, int32_t M, int32_t F, int32_t K, int32_t n_ctas, void* act,
+                   uint32_t* tile_flags, void* stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    if (M <= 0 || M > 128 || F <= 0 || K <= 0 || n_ctas <= 0 || path < 0 || path > 1) return OA_ERR_BAD_REQUEST;
+    CUtensorMap tmA, tmB;
+    if (!proj_maps(A, B, M, 2 * F, K, tmA, tmB)) return OA_ERR_INTERNAL;
+    DevBuf ws(streamk_ws_bytes(2 * F, 128, n_ctas, 128));
+    if (!ws.p) return OA_ERR_INTERNAL;
+    const StreamK sk = make_streamk((float*)ws.p, 2 * F, K, 128, n_ctas, 128);
+    cudaError_t e;
+    if (path == 0) {
+        e = launch_gemm_streamk(&tmA, &tmB, M, 2 * F, K, sk, s);
+        if (e == cudaSuccess) e = launch_sk_swiglu(sk, act, M, F, s);
+    } else {
+        e = launch_gemm_streamk_swiglu(&tmA, &tmB, M, F, K, sk, act, tile_flags, s);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    return rc_of(e);
+}
+
+int oa_k_qkv_rope(int32_t path, const void* A, const void* B, int32_t M, int32_t K, int32_t n_ctas, int32_t cluster, const void* bias,
+                  const int32_t* positions, const int32_t* slots, const float* rope_cos, const float* rope_sin, void* q_out, void* kv_cache,
+                  int32_t num_pages, int32_t n_layers, int32_t layer, int32_t nh, int32_t nkv, int32_t D, uint32_t* tile_flags, void* stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    const int N = (nh + 2 * nkv) * D;
+    if (M <= 0 || M > 128 || K <= 0 || n_ctas <= 0 || path < 0 || path > 3 || nh <= 0 || nkv <= 0 || (D != 64 && D != 128)) return OA_ERR_BAD_REQUEST;
+    if (n_layers < 1 || layer < 0 || layer >= n_layers) return OA_ERR_BAD_REQUEST;
+    if (path == 2 && (K + 63) / 64 < cluster) return OA_ERR_BAD_REQUEST;
+    KvLayout kv{}; kv.base = kv_cache; kv.page_size = 64; kv.n_kv = nkv; kv.head_dim = D; kv.num_pages = num_pages;
+    kv.kv_stride_rows = (int64_t)num_pages * nkv * 64; kv.layer_stride_rows = 2 * kv.kv_stride_rows;
+    CUtensorMap tmA, tmB;
+    if (!proj_maps(A, B, M, N, K, tmA, tmB)) return OA_ERR_INTERNAL;
+    cudaError_t e;
+    if (path == 3) {          // the tile GEMM's bf16 qkv tensor (+ bias), then RoPE + KV write from it
+        DevBuf qkv((size_t)M * N * 2);
+        if (!qkv.p) return OA_ERR_INTERNAL;
+        GemmParams g{}; g.M = M; g.N = N; g.K = K; g.out = qkv.p; g.ldo = N; g.bias = bias;
+        e = launch_gemm(&tmA, &tmB, g, EPI_STORE, 128, s);
+        if (e == cudaSuccess) e = launch_rope_kv_write(qkv.p, positions, slots, rope_cos, rope_sin, q_out, kv, layer, M, nh, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        return rc_of(e);
+    }
+    DevBuf ws(path == 2 ? 16 : streamk_ws_bytes(N, 128, n_ctas, 128));
+    if (!ws.p) return OA_ERR_INTERNAL;
+    const StreamK sk = make_streamk((float*)ws.p, N, K, 128, n_ctas, 128);
+    const SkRopeArgs ra = make_sk_rope_args(bias, positions, slots, rope_cos, rope_sin, q_out, kv, layer, nh);
+    if (path == 0) {
+        e = launch_gemm_streamk(&tmA, &tmB, M, N, K, sk, s);
+        if (e == cudaSuccess) e = launch_sk_rope_kv_write(sk, bias, positions, slots, rope_cos, rope_sin, q_out, kv, layer, M, nh, s);
+    } else if (path == 1) {
+        e = launch_gemm_streamk_rope(&tmA, &tmB, M, N, K, sk, ra, tile_flags, s);
+    } else {
+        e = launch_gemm_clusterk_rope(&tmA, &tmB, M, N, K, cluster, ra, s);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    return rc_of(e);
+}
+
+int oa_k_lm_head(const void* A, const void* B, int32_t M, int32_t N, int32_t K, int32_t block_n, const uint32_t* mask_table,
+                 const int32_t* mask_slot, int32_t mask_words, int32_t col_offset, float* logits, int32_t* ids, void* stream) {
+    cudaStream_t s = (cudaStream_t)stream;
+    if (M <= 0 || N <= 0 || K <= 0 || !ids) return OA_ERR_BAD_REQUEST;
+    CUtensorMap tmA, tmB;
+    if (make_tmap_bf16_2d(&tmA, A, (uint64_t)M, (uint64_t)K, (uint64_t)K, 128, 64) != 0) return OA_ERR_INTERNAL;
+    if (make_tmap_bf16_2d(&tmB, B, (uint64_t)N, (uint64_t)K, (uint64_t)K, (uint32_t)block_n, 64) != 0) return OA_ERR_INTERNAL;
+    const int nt = gemm_n_tiles(N, block_n);
+    DevBuf av((size_t)M * nt * 4), ai((size_t)M * nt * 4);
+    if (!av.p || !ai.p) return OA_ERR_INTERNAL;
+    GemmParams p{}; p.M = M; p.N = N; p.K = K; p.logits = logits; p.ldl = N; p.amax_val = (float*)av.p; p.amax_idx = (int*)ai.p;
+    p.mask_table = mask_table; p.mask_slot = mask_slot; p.mask_words = mask_words; p.col_offset = col_offset;
+    cudaError_t e = launch_gemm(&tmA, &tmB, p, EPI_LOGITS, block_n, s);
+    if (e == cudaSuccess) e = launch_argmax_reduce(p.amax_val, p.amax_idx, M, nt, ids, nullptr, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    return rc_of(e);
+}
+
 int oa_k_paged_attention(const void* q, void* out, const void* kv_cache, int32_t num_pages, const int32_t* block_tables,
                          int32_t max_pages_per_seq, const int32_t* ctx_lens, const int32_t* q_lens, int32_t n_seqs,
                          int32_t n_heads, int32_t n_kv, int32_t head_dim, int32_t force_splits, void* stream) {
+    return oa_k_paged_attention_ex(q, out, kv_cache, num_pages, 1, 0, block_tables, max_pages_per_seq, ctx_lens, q_lens, n_seqs, n_heads, n_kv,
+                                   head_dim, force_splits, 2 * 148, nullptr, stream);
+}
+
+int oa_k_paged_attention_ex(const void* q, void* out, const void* kv_cache, int32_t num_pages, int32_t n_layers, int32_t layer,
+                            const int32_t* block_tables, int32_t max_pages_per_seq, const int32_t* ctx_lens, const int32_t* q_lens, int32_t n_seqs,
+                            int32_t n_heads, int32_t n_kv, int32_t head_dim, int32_t force_splits, int32_t n_ctas_target, int32_t* merge_counters,
+                            void* stream) {
     cudaStream_t s = (cudaStream_t)stream;
+    if (n_layers < 1 || layer < 0 || layer >= n_layers) return OA_ERR_BAD_REQUEST;
     KvLayout kv{}; kv.base = const_cast<void*>(kv_cache); kv.page_size = 64; kv.n_kv = n_kv; kv.head_dim = head_dim; kv.num_pages = num_pages;
     kv.kv_stride_rows = (int64_t)num_pages * n_kv * 64; kv.layer_stride_rows = 2 * kv.kv_stride_rows;
-    CUtensorMap tm;
-    if (make_tmap_bf16_2d(&tm, kv_cache, (uint64_t)kv.layer_stride_rows, (uint64_t)head_dim, (uint64_t)head_dim, 64, 64) != 0) return OA_ERR_INTERNAL;
+    CUtensorMap tm;      // one map over every layer, as the engine builds it
+    if (make_tmap_bf16_2d(&tm, kv_cache, (uint64_t)kv.layer_stride_rows * n_layers, (uint64_t)head_dim, (uint64_t)head_dim, 64, 64) != 0) return OA_ERR_INTERNAL;
     const float scale_log2e = (1.0f / std::sqrt((float)head_dim)) * 1.4426950408889634f;
     const int grp = n_heads / n_kv;
     bool decode = true; int total_q = 0;
@@ -106,8 +228,9 @@ int oa_k_paged_attention(const void* q, void* out, const void* kv_cache, int32_t
     cudaMemcpyAsync(d_ctx.p, ctx_lens, (size_t)n_seqs * 4, cudaMemcpyHostToDevice, s);
     cudaError_t e;
     if (decode) {
+        if (n_ctas_target <= 0) n_ctas_target = 2 * device_sm_count();       // the engine's default: two CTAs per SM
         DecodePlan plan;
-        build_decode_plan(ctx_lens, n_seqs, n_kv, 2 * 148, force_splits, plan);
+        build_decode_plan(ctx_lens, n_seqs, n_kv, n_ctas_target, force_splits, plan);
         DevBuf d_segs(plan.segs.size() * sizeof(DecodeSeg)), d_ptr(plan.cta_ptr.size() * 4), d_merge(plan.merges.size() * sizeof(MergeItem));
         DevBuf d_po((size_t)(plan.n_slots + 1) * grp * head_dim * 4), d_pml((size_t)(plan.n_slots + 1) * grp * 2 * 4);
         if (!d_segs.p || !d_ptr.p || !d_merge.p || !d_po.p || !d_pml.p) return OA_ERR_INTERNAL;
@@ -116,10 +239,11 @@ int oa_k_paged_attention(const void* q, void* out, const void* kv_cache, int32_t
         cudaMemcpyAsync(d_merge.p, plan.merges.data(), plan.merges.size() * sizeof(MergeItem), cudaMemcpyHostToDevice, s);
         DecodeAttnParams a{}; a.q = q; a.out = out; a.block_tables = (const int32_t*)d_bt.p; a.ctx_lens = (const int32_t*)d_ctx.p;
         a.max_pages_per_seq = max_pages_per_seq; a.segs = (const DecodeSeg*)d_segs.p; a.cta_seg_ptr = (const int32_t*)d_ptr.p;
-        a.n_ctas = (int)plan.cta_ptr.size() - 1; a.part_o = (float*)d_po.p; a.part_ml = (float*)d_pml.p; a.layer = 0;
-        a.n_heads = n_heads; a.n_kv = n_kv; a.scale_log2e = scale_log2e;
+        a.n_ctas = (int)plan.cta_ptr.size() - 1; a.part_o = (float*)d_po.p; a.part_ml = (float*)d_pml.p; a.layer = layer;
+        a.n_heads = n_heads; a.n_kv = n_kv; a.scale_log2e = scale_log2e; a.merge_counters = merge_counters;
         e = launch_decode_attention(&tm, kv, a, s);
-        if (e == cudaSuccess) e = launch_decode_merge((const MergeItem*)d_merge.p, (int)plan.merges.size(), a.part_o, a.part_ml, out, n_heads, n_kv, head_dim, s);
+        if (e == cudaSuccess && !merge_counters)
+            e = launch_decode_merge((const MergeItem*)d_merge.p, (int)plan.merges.size(), a.part_o, a.part_ml, out, n_heads, n_kv, head_dim, s);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s);
         return rc_of(e);
     }
@@ -133,7 +257,7 @@ int oa_k_paged_attention(const void* q, void* out, const void* kv_cache, int32_t
     if (!d_tiles.p) return OA_ERR_INTERNAL;
     cudaMemcpyAsync(d_tiles.p, tiles.data(), tiles.size() * sizeof(PrefillTile), cudaMemcpyHostToDevice, s);
     PrefillAttnParams a{}; a.q = q; a.out = out; a.block_tables = (const int32_t*)d_bt.p; a.max_pages_per_seq = max_pages_per_seq;
-    a.tiles = (const PrefillTile*)d_tiles.p; a.n_tiles = (int)tiles.size(); a.layer = 0; a.n_heads = n_heads; a.n_kv = n_kv; a.scale_log2e = scale_log2e;
+    a.tiles = (const PrefillTile*)d_tiles.p; a.n_tiles = (int)tiles.size(); a.layer = layer; a.n_heads = n_heads; a.n_kv = n_kv; a.scale_log2e = scale_log2e;
     const char* leg = std::getenv("OA_PREFILL_ATTN");
     if (leg && std::string(leg) == "legacy") e = launch_prefill_attention(&tm, kv, a, s);
     else {
@@ -189,6 +313,8 @@ int oa_host_streamk_plan(int32_t N, int32_t K, int32_t block_n, int32_t n_ctas, 
     *n_ctas_out = sk.G; *n_tiles_out = sk.n_tiles; *kb_out = sk.kb;
     return OA_OK;
 }
+
+int32_t oa_host_clusterk_pick(int32_t N, int32_t K, int32_t sms, int32_t min_fill_pct) { return clusterk_pick(N, K, sms, min_fill_pct); }
 
 int oa_host_grammar_step(int32_t kind, const uint8_t* prefix, int32_t n, uint32_t* mask_out, int32_t* done_out) {
     return oa_host_grammar_step_ex(kind, "", prefix, n, mask_out, done_out);

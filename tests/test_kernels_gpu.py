@@ -10,6 +10,7 @@ pytestmark = pytest.mark.gpu
 
 from opsagent_b200 import _lib  # noqa: E402
 from oracle import oracle as O  # noqa: E402  (checker only)
+from oracle.attention_cases import AttnCase, assert_close, attn_tol  # noqa: E402
 
 EPI_STORE, EPI_RESID, EPI_SWIGLU, EPI_LOGITS = 0, 1, 2, 3
 
@@ -210,73 +211,50 @@ def test_gemm_streamk_partials_sum_to_the_product(L, M, N, K, G, bn):
 
 
 # ------------------------------------------------------------------------------------------------
-def _attn_ref(q, kcache, vcache, bt, ctx, qlens, nh, nkv, D):
-    """fp32 reference of paged causal GQA attention.  q: [sum(qlens), nh, D]"""
-    grp = nh // nkv
-    outs, row = [], 0
-    for i, (c, ql) in enumerate(zip(ctx, qlens)):
-        pages = bt[i, : (c + 63) // 64]
-        K = kcache[pages].permute(0, 2, 1, 3).reshape(-1, nkv, D)[:c].float()    # [c, nkv, D]
-        V = vcache[pages].permute(0, 2, 1, 3).reshape(-1, nkv, D)[:c].float()
-        qi = q[row:row + ql].float()                                              # [ql, nh, D]
-        Kh = K.repeat_interleave(grp, dim=1); Vh = V.repeat_interleave(grp, dim=1)
-        s = torch.einsum("qhd,khd->hqk", qi, Kh) / (D ** 0.5)
-        qpos = torch.arange(c - ql, c, device=q.device)[:, None]; kpos = torch.arange(c, device=q.device)[None, :]
-        s = s.masked_fill((kpos > qpos)[None], float("-inf"))
-        p = torch.softmax(s, dim=-1)
-        outs.append(torch.einsum("hqk,khd->qhd", p, Vh)); row += ql
-    return torch.cat(outs, 0)
-
-
-def _mk_cache(num_pages, nkv, D, seed):
-    g = torch.Generator(device="cpu").manual_seed(seed)
-    kv = torch.randn(2, num_pages, nkv, 64, D, generator=g).to(torch.bfloat16).to(dev())
-    return kv
+# attention inputs whose output depends on every 64-token chunk (oracle/attention_cases.py); fp64 reference, one bf16 ulp plus the
+# bound of the kernels' bf16 probabilities
+def _run_paged(L, ac, splits):
+    T = ac.q.shape[0]
+    out = torch.full((T, ac.nh, ac.D), float("nan"), dtype=torch.bfloat16, device=dev())
+    ctx_a = np.array(ac.ctx, np.int32); ql = np.array(ac.q_lens, np.int32); bt_np = np.ascontiguousarray(ac.bt.numpy())
+    rc = L.oa_k_paged_attention(ptr(ac.q), ptr(out), ptr(ac.kv[0]), ac.num_pages, bt_np.ctypes.data, ac.maxp, ctx_a.ctypes.data, ql.ctypes.data,
+                                len(ac.ctx), ac.nh, ac.nkv, ac.D, splits, None)
+    assert rc == 0, _lib.last_error()
+    return out
 
 
 @pytest.mark.parametrize("splits", [0, 3])
 @pytest.mark.parametrize("nh,nkv,D", [(32, 8, 128), (8, 2, 64), (5, 1, 64), (8, 1, 128), (40, 8, 128)])
 def test_paged_decode_attention(L, nh, nkv, D, splits):
     ctx = [1, 63, 64, 65, 200, 1000, 129, 517]
-    n = len(ctx); maxp = 20; num_pages = 150
-    kv = _mk_cache(num_pages, nkv, D, 11)
-    g = torch.Generator(device="cpu").manual_seed(5)
-    perm = torch.randperm(num_pages, generator=g)
-    bt = torch.zeros(n, maxp, dtype=torch.int32); k = 0
-    for i, c in enumerate(ctx):
-        npg = (c + 63) // 64; bt[i, :npg] = perm[k:k + npg].to(torch.int32); k += npg
-    q = torch.randn(n, nh, D, generator=g).to(torch.bfloat16).to(dev())
-    out = torch.full((n, nh, D), float("nan"), dtype=torch.bfloat16, device=dev())
-    ctx_a = np.array(ctx, np.int32); ql = np.ones(n, np.int32); bt_np = np.ascontiguousarray(bt.numpy())
-    rc = L.oa_k_paged_attention(ptr(q), ptr(out), ptr(kv), num_pages, bt_np.ctypes.data, maxp, ctx_a.ctypes.data, ql.ctypes.data, n,
-                                nh, nkv, D, splits, None)
-    assert rc == 0, _lib.last_error()
-    ref = _attn_ref(q, kv[0], kv[1], bt.to(dev()).long(), ctx, [1] * n, nh, nkv, D)
-    err = (out.float() - ref).abs().max().item()
-    assert torch.isfinite(out.float()).all()
-    assert err < 2e-2, err
+    ac = AttnCase(ctx, [1] * len(ctx), nh, nkv, D, n_layers=1, seed=11)
+    out = _run_paged(L, ac, splits)
+    ref, ref_abs = ac.ref(0)
+    tol = attn_tol(ref, ref_abs)
+    assert_close(out, ref, tol, "decode attention", max_frac=None)
+    ac.piece_power(0, ref, tol)
+
+
+@pytest.mark.parametrize("splits", [0, 3])
+@pytest.mark.parametrize("nh,nkv,D", [(32, 8, 128), (5, 1, 64)])
+def test_paged_decode_attention_flat(L, nh, nkv, D, splits):
+    """random q: the mass spreads over many keys and the running max keeps moving from chunk to chunk"""
+    ctx = [1, 65, 1000, 3000, 517]
+    ac = AttnCase(ctx, [1] * len(ctx), nh, nkv, D, n_layers=1, seed=13, flat=True)
+    out = _run_paged(L, ac, splits)
+    ref, ref_abs = ac.ref(0)
+    assert_close(out, ref, attn_tol(ref, ref_abs), "flat decode attention", max_frac=None)
 
 
 @pytest.mark.parametrize("nh,nkv,D", [(8, 2, 128), (4, 2, 64), (5, 1, 64)])
 def test_paged_prefill_attention(L, nh, nkv, D):
     # (ctx after the chunk, new rows): fresh prompts, a chunk continuing a cached prefix, ragged tile tails
     cases = [(64, 64), (130, 130), (200, 37), (1, 1), (333, 100), (128, 128)]
-    ctx = [c for c, _ in cases]; qlens = [q for _, q in cases]
-    n = len(ctx); maxp = 8; num_pages = 40
-    kv = _mk_cache(num_pages, nkv, D, 3)
-    g = torch.Generator(device="cpu").manual_seed(9)
-    perm = torch.randperm(num_pages, generator=g)
-    bt = torch.zeros(n, maxp, dtype=torch.int32); k = 0
-    for i, c in enumerate(ctx):
-        npg = (c + 63) // 64; bt[i, :npg] = perm[k:k + npg].to(torch.int32); k += npg
-    T = sum(qlens)
-    q = torch.randn(T, nh, D, generator=g).to(torch.bfloat16).to(dev())
-    out = torch.full((T, nh, D), float("nan"), dtype=torch.bfloat16, device=dev())
-    ctx_a = np.array(ctx, np.int32); ql = np.array(qlens, np.int32); bt_np = np.ascontiguousarray(bt.numpy())
-    rc = L.oa_k_paged_attention(ptr(q), ptr(out), ptr(kv), num_pages, bt_np.ctypes.data, maxp, ctx_a.ctypes.data, ql.ctypes.data, n,
-                                nh, nkv, D, 0, None)
-    assert rc == 0, _lib.last_error()
-    ref = _attn_ref(q, kv[0], kv[1], bt.to(dev()).long(), ctx, qlens, nh, nkv, D)
-    assert torch.isfinite(out.float()).all()
-    err = (out.float() - ref).abs().max().item()
-    assert err < 2e-2, err
+    for flat in (False, True):
+        ac = AttnCase([c for c, _ in cases], [q for _, q in cases], nh, nkv, D, n_layers=1, seed=3, flat=flat)
+        out = _run_paged(L, ac, 0)
+        ref, ref_abs = ac.ref(0)
+        tol = attn_tol(ref, ref_abs)
+        assert_close(out, ref, tol, f"prefill attention (flat={flat})", max_frac=None)
+        if not flat:
+            ac.piece_power(0, ref, tol)
